@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — rays/sec of the Instant-NGP hot path (BASELINE.json configs[1]: lego-shaped scene, 65 536 rays per batch).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (ray march -> hash/SH encode -> tiny MLPs -> alpha compositing) over one batch of
 65 536 synthetic Blender-shaped rays (800x800 spiral views, seeded lego-like occupancy grid, tcnn-default random weights).
@@ -175,7 +175,6 @@ def run_reference(args):
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
         return
-    t_start = time.time()
     sample_rays = 8192
     for _ in range(max(args.warmup, 1)):
         cpu_reference_rate(1024, reps=1)
@@ -185,8 +184,8 @@ def run_reference(args):
     for _ in range(args.steps):
         r, cores, kind, sample, dt = cpu_reference_rate(sample_rays, reps=1, threads=k_best)
         rates.append(r); per.append(dt)
-        if time.time() - t_start > 240:
-            break
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, cpu_reference_rate.last)
     value = float(np.median(rates))
     line = {
         'impl': 'reference', 'metric': METRIC, 'value': value, 'unit': 'rays/s', 'n_gpus': args.gpus, 'steps': len(rates), 'warmup': args.warmup,
@@ -350,6 +349,15 @@ def psnr_obj(a, b, what):
     return {'rays': int(a.shape[0]), 'max_abs_rgb_err': float(err.max()), 'psnr_vs_ref_db': float(-10.0 * np.log10(max(mse, 1e-20))), 'against': what}
 
 
+def dump_outputs(out_dir, last):
+    """--dump-outputs: what the headline path returned for the last timed batch (rank 0), as float32 .npy files, so that two builds run with the same
+    arguments (hence the same seeded rays, weights and jitter call index) can be compared output for output. The chain path also returns each ray's
+    sample base and the total sample count: those are the exclusive prefix sum and the sum of numsteps, which both paths return."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in zip(('rgb', 'alpha', 'numsteps'), last):
+        np.save(os.path.join(out_dir, name + '.npy'), np.asarray(t.cpu() if hasattr(t, 'cpu') else t, dtype=np.float32))
+
+
 # ------------------------------------------------------------------------------------------- our arm
 def run_ours(args):
     import torch
@@ -421,6 +429,7 @@ def run_ours(args):
     join()
     e1.record(main)
     barrier()
+    last_chain = (out[0].clone(), out[1].clone(), out[2][:, 0].clone())   # the renderer reuses its output buffers on the next call
     field_ms = [a.elapsed_time(b) for a, b in evf]
     samples = [int(c[1].item()) for c in counters_log]
     total_ms = float(e0.elapsed_time(e1))
@@ -505,6 +514,7 @@ def run_ours(args):
     join()
     f1.record(main)
     barrier()
+    last_fused = tuple(x.clone() for x in outf)
     if os.environ.get('XRB_BENCH_DEBUG') and kev:
         gaps = [evk[i][1].elapsed_time(evk[i + 1][0]) for i in range(K - 1)] if P == 1 else []
         kms = [a.elapsed_time(b) for a, b in evk]
@@ -518,6 +528,8 @@ def run_ours(args):
     fused_kernel_ms = float(np.mean([a.elapsed_time(b) for a, b in evk])) if kev else fused_total_ms / K
     fused_samples = float(np.mean([float(x.sum().item()) for x in ns_log]))
     use_fused = args.path == 'fused' or (args.path == 'auto' and fused_total_ms < total_ms_max)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_fused if use_fused else last_chain)
 
     # ---- end-to-end arm: host (pinned) rays in, rgb+alpha out, every step, through the public API; P batches in flight
     slots = [dict(rgb_h=torch.empty((N_RAYS, 3), dtype=torch.float32).pin_memory(), alpha_h=torch.empty((N_RAYS, 1), dtype=torch.float32).pin_memory(),
@@ -1085,6 +1097,8 @@ def main():
     ap.add_argument('--path', default='auto', choices=['auto', 'chain', 'fused'], help='inference path of the headline/e2e numbers: 5-launch chain, single-launch fused kernel, or the faster of the two (both are always measured)')
     ap.add_argument('--grad-comm', dest='grad_comm', default='auto', choices=['auto', 'peer', 'sharded', 'allreduce'], help='gradient exchange of the training arm at world > 1 (peer: one optimiser kernel over NVLink peer memory, csrc/peer_adam.cu; auto: peer where CUDA IPC works, else sharded NCCL)')
     ap.add_argument('--pipeline', type=int, default=8, help='ray batches in flight (CUDA streams); 1 = strictly sequential steps. Measured on one B200: 2 -> 240, 4 -> 271, 6 -> 287, 8 -> 292 M rays/s')
+    ap.add_argument('--dump-outputs', dest='dump_outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write rgb / alpha / numsteps of the headline path\'s last timed batch as DIR/<name>.npy (float32)')
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
     if args.impl == 'reference':

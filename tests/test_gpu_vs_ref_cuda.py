@@ -1,25 +1,24 @@
 """GPU cross-check against the REFERENCE's own CUDA kernels (extensions/ngp_raymarch built unmodified for sm_100a by oracle/build_ref_cuda.py), through the identical
-`raymarch_cuda` signatures. The bit-exact contract is defined on the un-contracted CPU build of the same sources (oracle/_ref, tests/test_gpu_raymarch.py): nvcc fuses
-the reference's `o + t*d` into FMAs, so here the march may differ in a handful of samples and the tolerances say so. Skipped when the module was not built."""
+`raymarch_cuda` signatures. What those kernels computed on a B200 for the inputs below is stored in tests/golden/raymarch_ref_cuda_golden.npz
+(tests/golden/make_golden_ref_cuda.py): per-ray sample counts, the samples of a fixed subset of the rays, and the composite of seeded raw values.
+The bit-exact contract is defined on the un-contracted CPU build of the same sources (oracle/_ref, tests/test_gpu_raymarch.py): nvcc fuses
+the reference's `o + t*d` into FMAs, so here the march may differ in a handful of samples and the tolerances say so."""
 import os
-import sys
 
 import numpy as np
 import pytest
 import torch
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'raymarch_ref_cuda_golden.npz')
+N_COORD_RAYS = 512      # rays whose samples the golden file keeps
+BG = (0.1, 0.2, 0.3)
 
 
 @pytest.fixture(scope='module')
-def ref():
-    sys.path.insert(0, ROOT)
-    from oracle import build_ref_cuda
-    m = build_ref_cuda.load_module()
-    if m is None:
-        pytest.skip('oracle/_ref/cuda/raymarch_cuda_ref.so not built')
-    return m
+def golden():
+    with np.load(GOLDEN) as z:
+        return {k: z[k] for k in z.files}
 
 
 @pytest.fixture(scope='module')
@@ -41,31 +40,51 @@ def _march(mod, o, d, bf, cap, ours_mod=None):
     return coords, ridx, ns, cnt
 
 
-def test_march_and_composite_agree_with_reference_cuda_kernels(ref, ours, scene):
+def scene_rays(scene):
     o = torch.from_numpy(np.ascontiguousarray(scene['rays_o'])).cuda(); d = torch.from_numpy(np.ascontiguousarray(scene['rays_d'])).cuda()
-    bf = torch.from_numpy(scene['bitfield']).cuda()
+    return o, d, torch.from_numpy(scene['bitfield']).cuda()
+
+
+def coord_rays(counts):
+    """a fixed sample of the rays the reference marched, whose samples are compared one by one"""
+    hit = np.nonzero(counts > 0)[0]
+    return np.sort(np.random.default_rng(3).choice(hit, min(len(hit), N_COORD_RAYS), replace=False))
+
+
+def composite_inputs(port, scene):
+    """the oracle's march of the scene's rays (bit-exact with ours, tests/test_gpu_raymarch.py) and seeded raw values"""
+    n = scene['rays_o'].shape[0]
+    c, _, ns, cnt = port.rays_sampler(scene['rays_o'], scene['rays_d'], scene['bitfield'], n * 256)
+    raw = (np.random.default_rng(21).standard_normal((int(cnt[1]), 4)) * 0.5).astype(np.float32)
+    return raw, np.ascontiguousarray(c[:cnt[1]]), ns
+
+
+def composite(mod, raw, coords, ns):
+    n = ns.shape[0]
+    rgb = torch.zeros((n, 3), device='cuda'); alpha = torch.zeros((n, 1), device='cuda')
+    mod.calc_rgb_influence_api(torch.from_numpy(raw).cuda(), torch.from_numpy(coords).cuda(), torch.from_numpy(ns).cuda(), torch.tensor(BG), 2, 3, 0.0, 1.0, rgb, alpha)
+    torch.cuda.synchronize()
+    return rgb.cpu().numpy(), alpha.cpu().numpy()
+
+
+def test_march_and_composite_agree_with_reference_cuda_kernels(golden, ours, port, scene):
+    o, d, bf = scene_rays(scene)
     n = o.shape[0]
-    cap = n * 256
-    cr, _, nr, cntr = _march(ref, o, d, bf, cap)              # first call of the process: the reference's static pcg32 is at its seed
-    co, _, no, cnto = _march(ours, o, d, bf, cap, ours)
-    a, b = nr[:, 0].cpu().numpy().astype(np.int64), no[:, 0].cpu().numpy().astype(np.int64)
-    assert abs(int(cntr[1]) - int(cnto[1])) <= max(8, int(cnto[1]) // 2000)
+    co, _, no, cnto = _march(ours, o, d, bf, n * 256, ours)
+    a, b = golden['ns'].astype(np.int64), no[:, 0].cpu().numpy().astype(np.int64)
+    assert abs(int(golden['cnt'][1]) - int(cnto[1])) <= max(8, int(cnto[1]) // 2000)
     assert (a != b).mean() < 2e-3                              # per-ray counts: all but FMA-rounding cases
-    same = np.nonzero((a == b) & (a > 0))[0][:2000]
-    br, bo = nr[:, 1].cpu().numpy(), no[:, 1].cpu().numpy()    # the reference's bases depend on atomic arrival order: compare ray by ray
-    crn, con = cr.cpu().numpy(), co.cpu().numpy()
-    worst = 0.0
-    for i in same:
-        worst = max(worst, float(np.abs(crn[br[i]:br[i] + a[i]] - con[bo[i]:bo[i] + a[i]]).max()))
+    rays = golden['rays']
+    assert np.array_equal(rays, coord_rays(a))
+    starts = np.concatenate([[0], np.cumsum(a[rays])])         # the golden samples of the kept rays, ray after ray
+    bo, con = no[:, 1].cpu().numpy(), co.cpu().numpy()
+    worst, compared = 0.0, 0
+    for j, i in enumerate(rays):
+        if a[i] == b[i]:
+            worst = max(worst, float(np.abs(golden['coords'][starts[j]:starts[j + 1]] - con[bo[i]:bo[i] + a[i]]).max()))
+            compared += 1
+    assert compared > len(rays) // 2
     assert worst <= 2e-6, worst                                 # positions differ by the FMA's one rounding at most
     # compositing of identical inputs through both kernels
-    s = int(cnto[1])
-    raw = torch.randn((s, 4), device='cuda') * 0.5
-    bg = torch.tensor([0.1, 0.2, 0.3])
-    out = []
-    for mod in (ref, ours):
-        rgb = torch.zeros((n, 3), device='cuda'); alpha = torch.zeros((n, 1), device='cuda')
-        mod.calc_rgb_influence_api(raw, co[:s].contiguous(), no, bg, 2, 3, 0.0, 1.0, rgb, alpha)
-        torch.cuda.synchronize()
-        out.append((rgb.clone(), alpha.clone()))
-    assert float((out[0][0] - out[1][0]).abs().max()) <= 2e-5 and float((out[0][1] - out[1][1]).abs().max()) <= 2e-5
+    rgb, alpha = composite(ours, *composite_inputs(port, scene))
+    assert float(np.abs(rgb - golden['rgb']).max()) <= 2e-5 and float(np.abs(alpha - golden['alpha']).max()) <= 2e-5

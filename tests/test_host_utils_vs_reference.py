@@ -1,32 +1,33 @@
-"""Host-side helpers of the networks against the REFERENCE's own functions, imported unmodified from /root/reference (this container only; skipped on the GPU box):
-batching.unfold_batching, transforms.recover_shape / merge_ret (networks/utils/batching.py:5-12, transforms.py:5-31), and NGPGridSampler.update_batch_rays
-(samplers/ngp_grid_sampler.py:268-284, restated: the reference class imports its CUDA extension at module import)."""
+"""Host-side helpers of the networks against the REFERENCE's own functions: batching.unfold_batching, transforms.recover_shape / merge_ret
+(networks/utils/batching.py:5-12, transforms.py:5-31), and NGPGridSampler.update_batch_rays (samplers/ngp_grid_sampler.py:268-284, restated: the reference
+class imports its CUDA extension at module import). The reference's outputs are stored in tests/golden/host_ref_golden.npz (tests/golden/make_golden_host.py)."""
 import math
 import os
 
+import numpy as np
 import pytest
 import torch
 
-pytestmark = pytest.mark.skipif(not os.path.isdir('/root/reference/xrnerf'), reason='needs /root/reference')
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'host_ref_golden.npz')
+N_UNFOLD = 5
 
 
-def _ref(name):
-    from oracle import ref_import as R
-    return R.load(name)
+@pytest.fixture(scope='module')
+def golden():
+    with np.load(GOLDEN) as z:
+        return {k: z[k] for k in z.files}
 
 
-def test_unfold_batching_recover_shape_merge_ret_match_reference():
+def test_unfold_batching_recover_shape_merge_ret_match_reference(golden):
     from xrnerf_b200.registry import networks as N
-    rb, rt = _ref('networks.utils.batching'), _ref('networks.utils.transforms')
-    g = torch.Generator().manual_seed(0)
-    for shape in [(1, 7, 3), (2, 5, 3), (3, 4), (6,), (1, 2, 4, 4)]:
-        x = torch.rand(shape, generator=g)
-        assert torch.equal(N.unfold_batching(x), rb.unfold_batching(x)), shape
-    data = torch.rand((12, 3), generator=g)
-    assert torch.equal(N.recover_shape(data, torch.tensor([3, 4, 3])), rt.recover_shape(data, torch.tensor([3, 4, 3])))
-    a = {k: torch.rand(5, generator=g) for k in ('rgb', 'disp', 'acc')}; b = {k: torch.rand(5, generator=g) for k in ('rgb', 'disp', 'acc')}
-    ours = N.merge_ret(dict(a), dict(b)); ref = rt.merge_ret(dict(a), dict(b))
-    assert set(ours) == set(ref) and all(torch.equal(ours[k], ref[k]) for k in ref)
+    G = {k: torch.from_numpy(v) for k, v in golden.items() if v.dtype.kind != 'U'}
+    for i in range(N_UNFOLD):
+        assert torch.equal(N.unfold_batching(G[f'unfold.{i}.x']), G[f'unfold.{i}.y']), G[f'unfold.{i}.x'].shape
+    assert torch.equal(N.recover_shape(G['recover.data'], G['recover.sizes']), G['recover.y'])
+    keys = ('rgb', 'disp', 'acc')
+    ours = N.merge_ret({k: G[f'merge.a.{k}'] for k in keys}, {k: G[f'merge.b.{k}'] for k in keys})
+    assert set(ours) == {k[len('merge.y.'):] for k in G if k.startswith('merge.y.')}
+    assert all(torch.equal(v, G['merge.y.' + k]) for k, v in ours.items())
 
 
 def test_update_batch_rays_rule():
@@ -49,22 +50,25 @@ def test_update_batch_rays_rule():
         assert smp.n_rays_per_batch == n0 and smp.measured_batch_size.item() == measured
 
 
-def test_reference_nerf_mlp_checkpoints_load_into_registry_modules():
-    """SURVEY 8f-4 (checkpoint compatibility): the state_dict of the REFERENCE's own NerfMLP (NeRF and Mip-NeRF embedders) has exactly our keys and shapes and loads
-    with strict=True; the packed tcgen05 weight image is rebuilt from the loaded weights."""
+def test_reference_nerf_mlp_checkpoints_load_into_registry_modules(golden):
+    """SURVEY 8f-4 (checkpoint compatibility): a state_dict laid out as the REFERENCE's own NerfMLP's (NeRF and Mip-NeRF embedders: keys in order, shapes,
+    input widths, as stored in the golden file) has exactly our keys and shapes and loads with strict=True; the packed tcgen05 weight image is rebuilt
+    from the loaded weights."""
     from xrnerf_b200 import registry as R
     from xrnerf_b200.nerf_mlp import pack_nerf_mlp_v3
-    mlpm = _ref('mlps.nerf_mlp'); _ref('embedders.base'); _ref('embedders.mipnerf_embedder')
     cfgs = [dict(skips=[4], netdepth=8, netwidth=256, output_ch=5, use_viewdirs=True, netchunk=1024 * 32, embedder=dict(type='BaseEmbedder', i_embed=0, multires=10, multires_dirs=4)),
             dict(skips=[4], netdepth=8, netwidth=256, use_viewdirs=True, netchunk=1024 * 32,
                  embedder=dict(type='MipNerfEmbedder', min_deg_point=0, max_deg_point=16, min_deg_view=0, max_deg_view=4, use_viewdirs=True, append_identity=True))]
-    for cfg in cfgs:
-        torch.manual_seed(0)
-        ref = mlpm.NerfMLP(**{k: (dict(v) if isinstance(v, dict) else v) for k, v in cfg.items()})
+    for i, cfg in enumerate(cfgs):
+        g = torch.Generator().manual_seed(i)
+        sd_ref = {}
+        for k, shape in zip(golden[f'mlp{i}.keys'].tolist(), golden[f'mlp{i}.shapes'].tolist()):
+            sd_ref[k] = torch.randn([s for s in shape if s], generator=g) * 0.05
+        sd_ref['pts_linears.0.bias'] = torch.from_numpy(golden[f'mlp{i}.pts_linears.0.bias'])
         ours = R.build_mlp(dict(cfg, type='NerfMLP'))
-        sd_ref, sd_ours = ref.state_dict(), ours.state_dict()
+        sd_ours = ours.state_dict()
         assert list(sd_ref) == list(sd_ours) and all(sd_ref[k].shape == sd_ours[k].shape for k in sd_ref)
-        assert (ref.input_ch, ref.input_ch_dirs) == (ours.input_ch, ours.input_ch_dirs)
+        assert (ours.input_ch, ours.input_ch_dirs) == tuple(golden[f'mlp{i}.input_ch'].tolist())
         ours.load_state_dict(sd_ref, strict=True)
         image, bias = pack_nerf_mlp_v3(ours)
         assert torch.equal(bias[:256], sd_ref['pts_linears.0.bias']) and image.numel() > 1_000_000

@@ -1,5 +1,5 @@
-"""Boundary tests: the reference's registry names / constructor kwargs / state_dict keys (SURVEY §8b, §5) and, where
-/root/reference is present, its config files loading unchanged. CPU for construction; GPU-marked for forward/train steps."""
+"""Boundary tests: the reference's registry names / constructor kwargs / state_dict keys (SURVEY §8b, §5) and the model entries
+of its config files (stored under tests/golden) loading unchanged. CPU for construction; GPU-marked for forward/train steps."""
 import os
 
 import numpy as np
@@ -47,15 +47,21 @@ def test_registry_names_and_state_dict_keys():
     assert mip.mlp.input_ch == 96 and mip.mlp.input_ch_dirs == 27
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/configs'), reason='reference configs only exist in the build container')
-def test_reference_config_files_load_unchanged():
+def test_reference_config_files_load_unchanged(tmp_path):
+    """every config of the three model families: its `model` entry and the last component of its `work_dir` (tests/golden/reference_configs.json, tests/golden/make_golden_host.py)
+    written back as a config file, loaded with the '#DATANAME#' substitution and built"""
+    import json
     from xrnerf_b200 import registry as R
-    for p, t in [('configs/nerf/nerf_blender_base01.py', 'NerfNetwork'), ('configs/nerf/nerf_llff_base01.py', 'NerfNetwork'), ('configs/instant_ngp/nerf_blender_local01.py', 'HashNerfNetwork'),
-                 ('configs/mipnerf/mipnerf_blender.py', 'MipNerfNetwork'), ('configs/mipnerf/mipnerf_multiscale.py', 'MipNerfNetwork')]:   # every config of the three model families
-        cfg = R.load_config(os.path.join('/root/reference', p), dataname='lego')
-        assert 'lego' in cfg.work_dir or 'lego' in str(cfg.get('basedata_cfg', ''))
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'reference_configs.json')) as fh:
+        configs = json.load(fh)
+    assert len(configs) == 5
+    for p, c in configs.items():
+        path = tmp_path / os.path.basename(p)
+        path.write_text(f'model = {c["model"]!r}\nwork_dir = {c["work_dir"]!r}\n')
+        cfg = R.load_config(str(path), dataname='lego')
+        assert 'lego' in cfg.work_dir
         net = R.build_network(cfg.model)
-        assert type(net).__name__ == t
+        assert type(net).__name__ == c['type'], p
 
 
 @pytest.mark.gpu
